@@ -1,17 +1,19 @@
 #!/usr/bin/env python
 """bench.py — Mbp decoded per second, one JSON line on rank 0.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--windows M] [--config 2|3] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--windows M] [--config 2|3] [--impl reference] [--dump-outputs DIR]
 
 Default (--config 2): BASELINE.json configs[1], synthetic 50 kb human-composition windows, --species=human ab initio.
 A "step" is one pass of the whole hot path (prep -> sweep -> backtrace -> pack) over the rank's batch of windows.  `value` is
-timed with CUDA events on the library's launch stream with the inputs already in HBM; `e2e` is the same metric through the public
-call (augb200_decode_batch) from host buffers, with the host->device copy of the windows and the device->host copy of the paths
-inside the timed region.  The job is world x M windows; no data-path collective; one NCCL gather of the final path arrays ends
-the e2e region.  After a first measurement the windows are re-dealt in proportion to each rank's measured sweep rate (the same
+timed with CUDA events on the library's launch stream with the inputs already in HBM over K steps; `e2e` is the same metric through
+the public call (augb200_decode_batch) from host buffers, with the host->device copy of the windows and the device->host copy of the
+paths inside the timed region, also over K steps.  The job is world x M windows; no data-path collective; one NCCL gather of the final
+path arrays ends each e2e step.  After a first measurement the windows are re-dealt in proportion to each rank's measured sweep rate (the same
 kernel runs up to 17 % slower on some GPUs of a node, SCALE_r01.json), `config.windows_per_gpu` lists the counts.
 The paths produced in the timed regions are checked against the reference's digests (tests/golden/ref_config2_digests.json):
 `verified` = number of windows compared, a mismatch aborts the run.
+`--dump-outputs DIR` writes the paths of the last device-resident step as float64 .npy files (dump_paths), so that two builds run
+with the same arguments can be compared output for output.
 
 --config 3: BASELINE.json configs[2], examples/chr2L in 157 windows of 200 kb, --species=fly defaults (UTR + softmasking +
 sample=100), windows sharded over the ranks; the same line layout.  The default run carries it under `secondary`.
@@ -303,6 +305,31 @@ def raw_tuples(raw, k):
     return [(int(pt[o + i]), int(pb[o + i]), int(pe[o + i]), int(ptr[o + i])) for i in range(n)]
 
 
+DUMP_BYTES = 63_000_000         # array data of --dump-outputs: with the .npy headers under 64 MB
+DUMP_SEED = 20261017
+
+
+def dump_paths(out_dir, window_ids, paths, budget=DUMP_BYTES, prefix=""):
+    """Write what a caller of the timed path receives, one float64 .npy per field: per window its global index (`window`), `status`,
+    `log_prob` and state count (`n_states`), and the condensed states of those windows concatenated in window order (`type`, `begin`,
+    `end`, `truncated`).  When all windows do not fit in `budget` bytes, windows are taken in a fixed seeded order while they fit and
+    written in index order; `window` says which."""
+    import numpy as np
+    cost = np.array([8 * (4 + 4 * len(p.states)) for p in paths], dtype=np.int64)       # 4 per-window values + 4 per state
+    keep = np.arange(len(paths))
+    if cost.sum() > budget:
+        order = np.random.default_rng(DUMP_SEED).permutation(len(paths))
+        keep = np.sort(order[:int(np.argmin(np.cumsum(cost[order]) <= budget))])
+    sel = [paths[k] for k in keep]
+    rows = np.array([(s.type, s.begin, s.end, s.truncated) for p in sel for s in p.states], dtype=np.float64).reshape(-1, 4)
+    arrays = {"window": np.asarray(window_ids, dtype=np.float64)[keep], "status": [p.status for p in sel],
+              "log_prob": [p.log_prob for p in sel], "n_states": [len(p.states) for p in sel],
+              "type": rows[:, 0], "begin": rows[:, 1], "end": rows[:, 2], "truncated": rows[:, 3]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def deal_windows(world, M, rates):
     """Window indices per rank: block-cyclic (window g -> rank g mod world), then the slower ranks hand their last windows to the
     faster ones so that the counts are proportional to the measured sweep rates.  Deterministic, the same on every rank."""
@@ -397,7 +424,13 @@ def main():
     ap.add_argument("--dropin-windows", type=int, default=2, help="chr2L windows of the drop-in end-to-end leg (0 = skip the leg)")
     ap.add_argument("--assume-rates", default="", help="testing only: comma-separated per-rank sweep rates to deal by instead of the measured ones")
     ap.add_argument("--no-balance", action="store_true", help="keep the block-cyclic deal (do not re-deal by measured sweep rate)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the paths of the last timed step (config 2) as DIR/<name>.npy, float64, "
+                                                          "at most 64 MB in all; with several GPUs each rank's files carry a rank<r>_ prefix")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != 2 or args.impl != "b200"):
+        ap.error("--dump-outputs writes the paths of the config-2 timed steps of --impl b200")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         reference_arm(args, rank, world)
@@ -592,6 +625,8 @@ def main():
     sweep_ms = dec.last_sweep_ms            # last run's sweep kernel, CUDA events around that launch
     assert all(p.status == 0 for p in paths)
     verified = verify_paths(lambda k: paths[k].as_tuples(), my_idx, digests)
+    if args.dump_outputs:
+        dump_paths(args.dump_outputs, my_idx, paths, DUMP_BYTES // world, "rank%d_" % rank if world > 1 else "")
     # ---- end-to-end through the public call, host buffers in, host paths out ----
     # untimed warm-up of the public call at full size (pinned + device buffers reach their final size; NCCL sets up its gather)
     raw = dec.decode_batch_raw(wins_b)
@@ -599,7 +634,7 @@ def main():
         shard.gather_to_rank0(shard.pack_paths(*raw), device="cuda")
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(1, min(args.steps, 2))
+    e2e_steps = args.steps
     d2h = 0
     for _ in range(e2e_steps):
         raw = dec.decode_batch_raw(wins_b)
@@ -707,7 +742,10 @@ def main():
             sec["dedup"] = {"unique_sampled_paths": uniq5, "path_states_all_samples": total5, "path_states_copied_to_host": int(len(samp5[4])),
                             "note": "k_pack_samples finds repeated state paths of a window on the device (SURVEY.md 8f next-1): only first occurrences cross PCIe"}
             if not args.no_cpu_baseline:
-                sec["cpu_baseline"] = calibrated_reference(n_per_proc=1, extra_args=("--sample=100", "--alternatives-from-sampling=true"))
+                try:
+                    sec["cpu_baseline"] = calibrated_reference(n_per_proc=1, extra_args=("--sample=100", "--alternatives-from-sampling=true"))
+                except RuntimeError as ex:          # no reference binary in this tree: the GPU measurement above still stands
+                    sec["cpu_baseline"] = {"error": repr(ex)}
             line["secondary"]["config5_sampling"] = sec
             dec.close()
         except Exception as ex:
@@ -723,7 +761,10 @@ def main():
             sec4 = {"workload": "%d x 200 kb synthetic windows, --species=human --UTR=on --softmasking=0 (71 states), 1 GPU, e2e from host buffers through augb200_decode_batch" % n4,
                     "value": n4 * l4 / 1e6 / dt4, "unit": "Mbp/s", "sweep_ms": dec4.last_sweep_ms, "path_states": int(out4[0].sum())}
             if not args.no_cpu_baseline:
-                sec4["cpu_baseline"] = calibrated_reference(n_per_proc=1, extra_args=("--UTR=on",), window_len=l4)
+                try:
+                    sec4["cpu_baseline"] = calibrated_reference(n_per_proc=1, extra_args=("--UTR=on",), window_len=l4)
+                except RuntimeError as ex:          # no reference binary in this tree: the GPU measurement above still stands
+                    sec4["cpu_baseline"] = {"error": repr(ex)}
             line["secondary"]["config4_utr"] = sec4
             dec4.close()
         except Exception as ex:
